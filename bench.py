@@ -227,12 +227,17 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-secondary', action='store_true', help='N=1: skip the C2 and C5-on-one-GPU legs')
     ap.add_argument('--sequences', type=int, default=C5_SEQUENCES, help='N>1: number of 4000-frame sequences')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='N=1: write the result arrays of the last timed step of the headline workload as DIR/<name>.npy '
+                         '(float64, inputs seeded: identical from run to run)')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
 
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
+    if args.dump_outputs and (args.impl != 'ours' or world > 1):
+        raise SystemExit('--dump-outputs writes the outputs of the one-GPU CUDA path (--impl ours, one process)')
 
     if args.impl == 'reference':
         run_reference(args, rank)
@@ -257,9 +262,25 @@ def main():
 # ------------------------------------------------------------------------------------------------------------------
 # N = 1
 # ------------------------------------------------------------------------------------------------------------------
-def time_job(model, pk, opts, obs, vis, args, chunk_len, flush, steps, warmup):
+RESULT_ARRAYS = ('fullpose', 'pose', 'trans', 'dmpls', 'markers_sim', 'errs', 'status', 'counters')
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as <out_dir>/<name>.npy, so that two builds can be compared output for output."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f'--dump-outputs: {total} bytes of outputs, more than {DUMP_LIMIT_BYTES}')
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
+
+
+def time_job(model, pk, opts, obs, vis, args, chunk_len, flush, steps, warmup, keep_outputs=False):
     """Device time of `steps` passes of the product's solve on one resident job: the launch over all chunks, the boundary
-    check and the repair launches (chmosh.launch_verified), each launch bracketed by CUDA events on the job's stream."""
+    check and the repair launches (chmosh.launch_verified), each launch bracketed by CUDA events on the job's stream.
+    ``keep_outputs``: also return, as float64 arrays, the result rows of the last timed pass (what job.download() hands
+    a caller)."""
     from moshpp_b200 import chmosh, lib
     prec = {'f32': lib.MOSH2_F32, 'f64': lib.MOSH2_F64}[args.precision]
     tol = chmosh.BOUNDARY_TOL['fast']
@@ -284,6 +305,10 @@ def time_job(model, pk, opts, obs, vis, args, chunk_len, flush, steps, warmup):
         launches += len(rep['kernel_ms'])
     wall = time.perf_counter() - t0
     totals = job.totals()
+    outputs = None
+    if keep_outputs:          # copies: the end-to-end leg below reuses the job's result buffers
+        last = job.download()
+        outputs = {k: np.array(getattr(last, k), dtype=np.float64) for k in RESULT_ARRAYS}
     # C-ABI job-level end to end: pinned H2D + launches + D2H of all result arrays
     e2e = []
     for i in range(2 + steps):
@@ -294,7 +319,7 @@ def time_job(model, pk, opts, obs, vis, args, chunk_len, flush, steps, warmup):
     solved = int(((res.status & lib.ST_SOLVED) != 0).sum())
     out = dict(ms=float(np.mean(ms)), first_launch_ms=float(np.mean(first_ms)), e2e_job_ms=float(np.mean(e2e)) * 1e3, totals=totals,
                chunks=job.num_chunks, chunk_len=chunk_len, first_extra=extra, solved=solved, wall=wall, flags=int(np.bitwise_or.reduce(res.status)), launches=launches,
-               boundary=rep)
+               boundary=rep, outputs=outputs)
     job.close()
     return out
 
@@ -343,7 +368,10 @@ def run_single(args):
     obs, vis = dense(case)
     F = obs.shape[0]
     model = lib.Model(pk, device=dev)
-    ns = time_job(model, pk, opts, obs, vis, args, args.chunk_len, flush, args.steps, args.warmup)
+    ns = time_job(model, pk, opts, obs, vis, args, args.chunk_len, flush, args.steps, args.warmup,
+                  keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ns['outputs'])
     chunk_len = ns['chunk_len']
     e2e_ms, out, e2e_each, e2e_cold = time_plugin(case, args, args.steps, 2, chunk_len=args.chunk_len)
     b = out['stageii_debug_details']['b200']

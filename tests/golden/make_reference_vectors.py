@@ -13,6 +13,9 @@
     exclusion and the collinear-neighbour fallback) and `TransformedLms` (simulated markers on posed vertices)
     -> ref_prior.npz, ref_lms.npz.
 
+  * scan2mesh/mesh_distance/sample2meshdist.h (row f-2), compiled unmodified by oracle/build_ref.py: the
+    point-to-triangle distance and its gradients -> ref_s2m.npz.
+
 The vectors travel with the repository; /root/reference is needed only to regenerate them:
 
     python tests/golden/make_reference_vectors.py
@@ -166,6 +169,36 @@ def prior_and_marker_vectors():
     print('ref_lms.npz:', {k: v.shape for k, v in cases.items() if k.startswith('closest')})
 
 
+def mesh_distance_vectors():
+    """Row f-2: the point-to-triangle distance of scan2mesh/mesh_distance/sample2meshdist.h, UNMODIFIED, compiled against
+    the Eigen stand-in (oracle/build_ref.py): value and the four gradients of every part (plane, three edges, three
+    vertices) under the three robustifiers on 40 random (sample, triangle) cases -> ref_s2m.npz."""
+    import ctypes as C
+    from oracle import build_ref
+    from oracle import mesh_distance as omd
+
+    lib = C.CDLL(build_ref.build(force=True))
+    dp = C.POINTER(C.c_double)
+    lib.s2m_tri.restype = C.c_double
+    lib.s2m_tri.argtypes = [C.c_int, C.c_double, C.c_int, dp, dp, dp, dp, dp, dp, dp, dp]
+    rng = np.random.default_rng(7)
+    kinds = np.array([(omd.KIND_DISTANCE, 1.0), (omd.KIND_SQUARED, 1.0), (omd.KIND_GM, 0.05), (omd.KIND_GM, 0.5)])
+    xabc = np.zeros((40, 4, 3))
+    value, grad = np.zeros((40, len(kinds), 7)), np.zeros((40, len(kinds), 7, 4, 3))
+    for t in range(40):
+        a, b, c = rng.normal(0, 0.3, (3, 3))
+        xabc[t] = (a + b + c) / 3 + rng.normal(0, 0.2, 3), a, b, c
+        for k, (kind, sigma) in enumerate(kinds):
+            for part in range(7):
+                args = [np.ascontiguousarray(v) for v in xabc[t]]
+                bufs = [np.zeros(3) for _ in range(4)]
+                value[t, k, part] = lib.s2m_tri(int(kind), float(sigma), part, *[v.ctypes.data_as(dp) for v in args + bufs])
+                grad[t, k, part] = bufs
+    np.savez_compressed(os.path.join(HERE, 'ref_s2m.npz'), kinds=kinds, xabc=xabc, value=value, grad=grad)
+    print('ref_s2m.npz:', value.shape, grad.shape)
+
+
 if __name__ == '__main__':
     main()
     prior_and_marker_vectors()
+    mesh_distance_vectors()

@@ -1,36 +1,17 @@
 """Stage-I surface term (SURVEY.md 8(f-2)): point-to-triangle-mesh distance with derivatives.
 
-CPU: the oracle's restatement against the reference header itself (oracle/_ref/libs2m.so = the UNMODIFIED
-scan2mesh/mesh_distance/sample2meshdist.h compiled against an Eigen stand-in, oracle/build_ref.py) and against finite
-differences.  GPU: the CUDA kernel (C-ABI mosh2_mesh_distance) against the oracle."""
-import ctypes as C
+CPU: the oracle's restatement against the reference header itself (values of the UNMODIFIED
+scan2mesh/mesh_distance/sample2meshdist.h compiled against an Eigen stand-in, stored in tests/golden/ref_s2m.npz by
+tests/golden/make_reference_vectors.py) and against finite differences.  GPU: the CUDA kernel (C-ABI
+mosh2_mesh_distance) against the oracle."""
 import os
 
 import numpy as np
 import pytest
 
-from oracle import build_ref
 from oracle import mesh_distance as omd
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-@pytest.fixture(scope='module')
-def s2m():
-    path = build_ref.build()
-    if not path:
-        pytest.skip('oracle/_ref/libs2m.so is not built and /root/reference is not present')
-    lib = C.CDLL(path)
-    dp = C.POINTER(C.c_double)
-    lib.s2m_tri.restype = C.c_double
-    lib.s2m_tri.argtypes = [C.c_int, C.c_double, C.c_int, dp, dp, dp, dp, dp, dp, dp, dp]
-
-    def tri(kind, sigma, part, x, a, b, c):
-        bufs = [np.zeros(3) for _ in range(4)]
-        args = [np.ascontiguousarray(v, dtype=np.float64) for v in (x, a, b, c)]
-        val = lib.s2m_tri(kind, sigma, part, *[v.ctypes.data_as(dp) for v in args], *[v.ctypes.data_as(dp) for v in bufs])
-        return (val, *bufs)
-    return tri
 
 
 def _random_case(rng):
@@ -39,18 +20,18 @@ def _random_case(rng):
     return x, a, b, c
 
 
-def test_oracle_tri_equals_reference_header(s2m):
+def test_oracle_tri_equals_reference_header():
     """Every part (plane, three edges, three vertices) under the three robustifiers: value and all four gradients."""
-    rng = np.random.default_rng(7)
-    for trial in range(40):
-        x, a, b, c = _random_case(rng)
-        for kind, sigma in ((omd.KIND_DISTANCE, 1.0), (omd.KIND_SQUARED, 1.0), (omd.KIND_GM, 0.05), (omd.KIND_GM, 0.5)):
+    g = np.load(os.path.join(ROOT, 'tests', 'golden', 'ref_s2m.npz'))
+    assert g['xabc'].shape[0] == 40 and len(g['kinds']) == 4
+    for trial, (x, a, b, c) in enumerate(g['xabc']):
+        for k, (kind, sigma) in enumerate(g['kinds']):
             for part in range(7):
-                ref = s2m(kind, sigma, part, x, a, b, c)
-                got = omd.tri(part, x, a, b, c, kind, sigma)
+                ref = (g['value'][trial, k, part], *g['grad'][trial, k, part])
+                got = omd.tri(part, x, a, b, c, int(kind), float(sigma))
                 assert abs(got[0] - ref[0]) <= 1e-12 * max(1.0, abs(ref[0]))
-                for g, r in zip(got[1:], ref[1:]):
-                    assert np.abs(g - r).max() <= 1e-10 * max(1.0, np.abs(r).max()), (kind, part)
+                for gr, r in zip(got[1:], ref[1:]):
+                    assert np.abs(gr - r).max() <= 1e-10 * max(1.0, np.abs(r).max()), (kind, part)
 
 
 def test_oracle_gradients_are_derivatives():
