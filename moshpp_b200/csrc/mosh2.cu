@@ -9,7 +9,6 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
-#include <algorithm>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -174,96 +173,7 @@ struct DevModel {
         return 0;
     }
     int build(const mosh2_model_desc &d) {
-        const size_t nJ = d.n_joints, S = size_t(3) * d.n_markers, nd = d.n_dmpl;
-        m.nJ = d.n_joints; m.M = d.n_markers; m.body_dof = d.body_dof; m.p_red = d.p_red;
-        m.n_hand_red = d.n_hand_red; m.n_hand_full = d.n_hand_full; m.nd = d.n_dmpl; m.kw = d.kw;
-        m.prior_k = d.prior_k; m.prior_d = d.prior_d;
-        m.n1 = d.n_free1; m.n2 = d.n_free2; m.finger_lo = d.finger_lo; m.finger_hi = d.finger_hi;
-        m.n_expr = d.n_expr; m.face_lo = d.face_lo; m.face_hi = d.face_hi;
-        m.n_jang = d.n_jangles;
-        for (int i = 0; i < d.n_jangles && i < mosh2::kMaxJangles; ++i) { m.jang_id[i] = d.jangles_ids[i]; m.jang_sign[i] = real(d.jangles_signs[i]); }
-        int rc;
-        if ((rc = up<int>(d.parents, nJ, &m.parents))) return rc;
-        std::vector<int> order(nJ), ids(d.prior_d);
-        std::vector<double> hct;
-        {   // joints sorted by depth (stable): parents before children
-            std::vector<int> depth(nJ, 0);
-            for (size_t j = 0; j < nJ; ++j) { int dj = 0; for (int a = d.parents[j]; a >= 0; a = d.parents[a]) ++dj; depth[j] = dj; }
-            for (size_t j = 0; j < nJ; ++j) order[j] = int(j);
-            std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return depth[a] < depth[b]; });
-            if ((rc = up<int>(order.data(), nJ, &m.fk_order))) return rc;
-        }
-        if ((rc = up<int>(d.w_joint, S * d.kw, &m.w_joint))) return rc;
-        {   // dense blocks of the hand-PCA matrix (rows with the same non-zero column range), stored transposed
-            mosh2::HandBlock blocks[mosh2::kMaxHandBlocks];
-            const int nb = mosh2_host::hand_blocks(d.hand_comps, d.n_hand_red, d.n_hand_full, blocks, hct);
-            m.hb_n = nb;
-            for (int b = 0; b < nb; ++b) m.hb[b] = blocks[b];
-            m.hct_size = int(hct.size());
-            if ((rc = up<real>(hct.data(), hct.size(), &m.hct))) return rc;
-        }
-        if ((rc = up<real>(d.hands_mean, d.n_hand_full, &m.hands_mean))) return rc;
-        if ((rc = up<real>(d.v0, S * 3, &m.v0))) return rc;
-        if ((rc = up<real>(d.sd, S * 3 * nd, &m.sd))) return rc;
-        {   // pose-blend table twice: [(nJ-1)][9 e][3 c][Sp] (eval: four slots per 16-byte load, no padding) and
-            // [(nJ-1)][9 e][3M slots][x y z -] (build: one slot per 16-byte load)
-            const size_t S3 = size_t(3) * d.n_markers;
-            const size_t Sp = (S3 + 3) & ~size_t(3);
-            std::vector<double> pdc((nJ - 1) * 27 * Sp, 0.0), pd4((nJ - 1) * 9 * S3 * 4, 0.0);
-            for (size_t j = 0; j + 1 < nJ; ++j)
-                for (size_t sl = 0; sl < S3; ++sl)
-                    for (int c = 0; c < 3; ++c)
-                        for (int e = 0; e < 9; ++e) {
-                            const double v = d.pd[(j * 3 * S3 + 3 * sl + c) * 9 + e];
-                            pdc[((j * 9 + e) * 3 + c) * Sp + sl] = v;
-                            pd4[((j * 9 + e) * S3 + sl) * 4 + c] = v;
-                        }
-            if ((rc = up<real>(pdc.data(), pdc.size(), &m.pdc))) return rc;
-            if ((rc = up<real>(pd4.data(), pd4.size(), &m.pd4))) return rc;
-        }
-        if ((rc = up<real>(d.w_val, S * d.kw, &m.w_val))) return rc;
-        if ((rc = up<real>(d.j0, nJ * 3, &m.j0))) return rc;
-        if ((rc = up<real>(d.jd, nJ * 3 * nd, &m.jd))) return rc;
-        if ((rc = up<real>(d.coefs, size_t(d.n_markers) * 3, &m.coefs))) return rc;
-        if ((rc = up<real>(d.prior_means, size_t(d.prior_k) * d.prior_d, &m.prior_means))) return rc;
-        {
-            const size_t K = d.prior_k, D = d.prior_d, D4 = (D + 3) & ~size_t(3);
-            m.prior_d4 = int(D4);
-            std::vector<double> q4(K * D * D4, 0.0);
-            for (size_t k = 0; k < K; ++k)
-                for (size_t i = 0; i < D; ++i)
-                    for (size_t l = 0; l < D; ++l) q4[(k * D + i) * D4 + l] = d.prior_Q[(k * D + i) * D + l];
-            if ((rc = up<real>(q4.data(), q4.size(), &m.prior_Q4))) return rc;
-            std::vector<double> qt(K * D * D4, 0.0);
-            for (size_t k = 0; k < K; ++k)
-                for (size_t i = 0; i < D; ++i)
-                    for (size_t l = 0; l < D; ++l) qt[(k * D + l) * D4 + i] = d.prior_Q[(k * D + i) * D + l];
-            if ((rc = up<real>(qt.data(), qt.size(), &m.prior_Qt))) return rc;
-        }
-        if ((rc = up<real>(d.prior_neglogw, d.prior_k, &m.prior_nlw))) return rc;
-        {
-            for (int i = 0; i < d.prior_d; ++i) ids[i] = d.prior_ids ? d.prior_ids[i] : d.prior_off + i;
-            if ((rc = up<int>(ids.data(), ids.size(), &m.prior_ids))) return rc;
-        }
-        if ((rc = up<int>(d.free1, d.n_free1, &m.free1))) return rc;
-        if ((rc = up<int>(d.free2, d.n_free2, &m.free2))) return rc;
-        {   // image of the staged shared-memory tables (mosh2::carve / stage_image): what a chunk fetches with one bulk copy
-            const mosh2::Dims dd = mosh2::make_dims(m);
-            mosh2::Work<real, false> w{};
-            mosh2::Arena S{mosh2::kSmemHeader}, G{0};
-            mosh2::carve<real, false>(w, dd, m, S, G);
-            std::vector<unsigned char> img(w.stage_bytes, 0);
-            const int *isrc[6] = {d.parents, order.data(), d.w_joint, d.free1, d.free2, ids.data()};
-            const double *rsrc[9] = {d.w_val, d.v0, d.coefs, d.j0, d.hands_mean, d.prior_means, d.prior_neglogw, d.jd, hct.data()};
-            mosh2::stage_image(w, dd, m.hct_size, m.n_hand_full, [&](uint32_t ofs, int id, size_t n) {
-                if (id < 6) { int *o = reinterpret_cast<int *>(img.data() + ofs); for (size_t i = 0; i < n; ++i) o[i] = isrc[id][i]; }
-                else { real *o = reinterpret_cast<real *>(img.data() + ofs); for (size_t i = 0; i < n; ++i) o[i] = real(rsrc[id - 6][i]); }
-            });
-            const unsigned char *blob = nullptr;
-            if ((rc = up<unsigned char>(img.data(), img.size(), &blob))) return rc;
-            m.stage_blob = blob;
-        }
-        return 0;
+        return mosh2_host::build_model(d, m, [this](const auto *src, size_t n, auto **dst) { return up(src, n, dst); });
     }
 };
 
@@ -404,7 +314,7 @@ struct mosh2_model {
 struct mosh2_job {
     mosh2_model *model = nullptr;
     int precision = MOSH2_F32;
-    int n_frames = 0, chunk_len = 0, warmup = 0, warm_full = 0, n_chunks = 1;
+    int n_frames = 0, n_chunks = 1;
     int *d_chunk_tab = nullptr, *d_chunk_ids = nullptr, *d_warm_f = nullptr;
     void *d_warm_x = nullptr;
     float *d_delta = nullptr;
@@ -611,23 +521,14 @@ int mosh2_job_create_batch(mosh2_model *m, const mosh2_options *opt, int32_t n_s
     mosh2_job *j = new (std::nothrow) mosh2_job;
     if (!j) return fail(MOSH2_E_INVALID, "out of host memory");
     j->model = m; j->precision = precision; j->n_frames = n_frames;
-    const int chunk_len = sched ? sched->chunk_len : 0, chunk_warmup = sched ? sched->chunk_warmup : 0;
-    j->chunk_len = chunk_len > 0 ? chunk_len : 0;
-    j->warmup = chunk_warmup > 0 ? chunk_warmup : 0;
-    j->warm_full = (!sched || sched->warmup_full < 0 || sched->warmup_full > j->warmup) ? j->warmup : sched->warmup_full;
-    const int first_extra = (sched && sched->first_extra > 0 && j->chunk_len > 0 && j->warmup > 0) ? sched->first_extra : 0;
-    j->tab = mosh2_host::chunk_table(frame_counts, n_seq, j->chunk_len, j->warmup, j->warm_full, first_extra);
+    const mosh2_host::Schedule s = mosh2_host::schedule(sched);
+    j->tab = mosh2_host::chunk_table(frame_counts, n_seq, s.chunk_len, s.warmup, s.warm_full, s.first_extra);
     j->tab0 = j->tab;
     const std::vector<int> &tab = j->tab;
     j->n_chunks = int(tab.size() / mosh2::kChunkRec);
     j->launch_blocks = j->n_chunks;
     j->esz = precision == MOSH2_F64 ? 8 : 4;
-    mosh2::Options &o = j->opt;
-    o.wt_data = opt->wt_data; o.wt_poseB = opt->wt_poseB; o.wt_poseH = opt->wt_poseH; o.wt_velo = opt->wt_velo;
-    o.wt_dmpl = opt->wt_dmpl; o.wt_annealing = opt->wt_annealing; o.wt_extrap = opt->wt_extrap_dmpl;
-    o.num_train_markers = opt->num_train_markers; o.delta_0 = opt->delta_0; o.e3_first = opt->e3_first; o.e3 = opt->e3;
-    o.maxiter = opt->maxiter; o.optimize_fingers = opt->optimize_fingers; o.optimize_dynamics = opt->optimize_dynamics;
-    o.wt_poseF = opt->wt_poseF; o.wt_expr = opt->wt_expr; o.optimize_face = opt->optimize_face;
+    j->opt = mosh2_host::options(opt);
 
     size_t gws = 0;
     if (precision == MOSH2_F64) plan_workspace(m->f64.m, &j->smem, &gws, &j->big_in_global);
@@ -805,7 +706,7 @@ int mosh2_job_relaunch_chunks(mosh2_job *j, int32_t n, const int32_t *chunk_ids,
     if (!j || n < 1 || !chunk_ids || !(merge_tol >= 0)) return fail(MOSH2_E_INVALID, "bad argument");
     j->merge_tol = merge_tol;
     CU(cudaSetDevice(j->model->device));
-    const int wf = chunk_warmup < 0 ? 0 : ((warmup_full < 0 || warmup_full > chunk_warmup) ? chunk_warmup : warmup_full);
+    const int wf = chunk_warmup < 0 ? 0 : mosh2_host::clamp_warm_full(chunk_warmup, warmup_full);
     for (int k = 0; k < n; ++k) {
         const int c = chunk_ids[k];
         if (c < 0 || c >= j->n_chunks) return fail(MOSH2_E_INVALID, "chunk %d out of range (%d chunks)", c, j->n_chunks);

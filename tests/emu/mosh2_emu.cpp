@@ -8,7 +8,6 @@
 #include "../../moshpp_b200/csrc/mosh2_device.cuh"
 #include "../../moshpp_b200/csrc/mosh2_host.h"
 
-#include <algorithm>
 #include <cstdlib>
 #include <cstdio>
 #include <cstring>
@@ -16,103 +15,72 @@
 
 namespace {
 
+// One job on the single "thread block": the model tables as libmosh2.so builds them (mosh2_host::build_model), kept in host
+// memory, the job's output rows, and the shared-memory buffer each chunk runs on.
 template <class real>
-struct HostModel {
+struct Emu {
     mosh2::Model<real> m{};
-    std::vector<std::vector<char>> store;
+    mosh2::Job<real> job{};
+    std::vector<std::vector<char>> tables;
+    std::vector<real> fullpose, pose, trans, dmpls, mk, errs;
+    std::vector<int> status, counters;
+    mosh2::Dims d{};
+    mosh2::Work<real, false> w{};
+    size_t smem_bytes = 0;
+    std::vector<char> smem_raw;
+
     template <class T, class U>
-    const T *up(const U *src, size_t n) {
-        store.emplace_back((n + 1) * sizeof(T) + 32);
-        char *raw = store.back().data();
+    int up(const U *src, size_t n, const T **dst) {
+        tables.emplace_back((n + 1) * sizeof(T) + 32);
+        char *raw = tables.back().data();
         T *p = reinterpret_cast<T *>(raw + ((32 - (reinterpret_cast<uintptr_t>(raw) & 31)) & 31));
         for (size_t i = 0; i < n; ++i) p[i] = static_cast<T>(src[i]);
-        return p;
+        *dst = p;
+        return 0;
     }
-    void build(const mosh2_model_desc &d) {
-        const size_t nJ = d.n_joints, S = size_t(3) * d.n_markers, nd = d.n_dmpl;
-        m.nJ = d.n_joints; m.M = d.n_markers; m.body_dof = d.body_dof; m.p_red = d.p_red;
-        m.n_hand_red = d.n_hand_red; m.n_hand_full = d.n_hand_full; m.nd = d.n_dmpl; m.kw = d.kw;
-        m.prior_k = d.prior_k; m.prior_d = d.prior_d;
-        m.n1 = d.n_free1; m.n2 = d.n_free2; m.finger_lo = d.finger_lo; m.finger_hi = d.finger_hi;
-        m.n_expr = d.n_expr; m.face_lo = d.face_lo; m.face_hi = d.face_hi;
-        m.n_jang = d.n_jangles;
-        for (int i = 0; i < d.n_jangles && i < mosh2::kMaxJangles; ++i) { m.jang_id[i] = d.jangles_ids[i]; m.jang_sign[i] = real(d.jangles_signs[i]); }
-        m.parents = up<int>(d.parents, nJ);
-        {
-            std::vector<int> depth(nJ, 0), order(nJ);
-            for (size_t j = 0; j < nJ; ++j) { int dj = 0; for (int a = d.parents[j]; a >= 0; a = d.parents[a]) ++dj; depth[j] = dj; }
-            for (size_t j = 0; j < nJ; ++j) order[j] = int(j);
-            std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return depth[a] < depth[b]; });
-            m.fk_order = up<int>(order.data(), nJ);
+
+    Emu(const mosh2_model_desc &desc, const mosh2_options *opt, int n_frames) {
+        mosh2_host::build_model(desc, m, [this](const auto *src, size_t n, auto **dst) { return up(src, n, dst); });
+        if (std::getenv("MOSH2_EMU_PLAN")) {        // development aid: shared-memory footprint of this model
+            for (int tile : {20, 10}) {
+                m.tile_markers = tile;
+                m.dev_no_tc = sizeof(real) == 4 ? 0 : 1;   // what the GPU launch would lay out
+                const mosh2::Dims dd = mosh2::make_dims(m);
+                mosh2::Work<real, false> ww{};
+                mosh2::Arena Sa{mosh2::kSmemHeader}, Ga{0};
+                mosh2::carve<real, false>(ww, dd, m, Sa, Ga);
+                std::fprintf(stderr, "plan: sizeof(real)=%zu tile=%d smem=%zu bytes (limit %d)\n", sizeof(real), tile, Sa.off, 227 * 1024);
+                std::fprintf(stderr, "      A=%u Lm=%u Xhi=%u Xlo=%u Jt=%u Jf=%u Loc=%u MtR=%u u=%u dtg=%u Linv=%u tc_ok=%d\n", ww.A.ofs, ww.Lm.ofs, ww.Xhi.ofs,
+                             ww.Xlo.ofs, ww.Jt.ofs, ww.Jf.ofs, ww.Loc.ofs, ww.MtR.ofs, ww.u.ofs, ww.dtg.ofs, ww.Linv.ofs, ww.tc_ok);
+            }
         }
-        m.w_joint = up<int>(d.w_joint, S * d.kw);
-        {
-            std::vector<double> hct;
-            mosh2::HandBlock blocks[mosh2::kMaxHandBlocks];
-            m.hb_n = mosh2_host::hand_blocks(d.hand_comps, d.n_hand_red, d.n_hand_full, blocks, hct);
-            for (int b = 0; b < m.hb_n; ++b) m.hb[b] = blocks[b];
-            m.hct_size = int(hct.size());
-            m.hct = up<real>(hct.data(), hct.size());
-        }
-        m.hands_mean = up<real>(d.hands_mean, d.n_hand_full);
-        m.v0 = up<real>(d.v0, S * 3);
-        m.sd = up<real>(d.sd, S * 3 * nd);
-        {
-            // [(nJ-1)][9 e][3M slots][4]: x, y, z of a slot for one (joint, e) form one 16-byte vector
-            const size_t S3 = size_t(3) * d.n_markers;
-            const size_t Sp = (S3 + 3) & ~size_t(3);
-            std::vector<double> pdc((nJ - 1) * 27 * Sp, 0.0), pd4((nJ - 1) * 9 * S3 * 4, 0.0);
-            for (size_t j = 0; j + 1 < nJ; ++j)
-                for (size_t sl = 0; sl < S3; ++sl)
-                    for (int c = 0; c < 3; ++c)
-                        for (int e = 0; e < 9; ++e) {
-                            const double v = d.pd[(j * 3 * S3 + 3 * sl + c) * 9 + e];
-                            pdc[((j * 9 + e) * 3 + c) * Sp + sl] = v;
-                            pd4[((j * 9 + e) * S3 + sl) * 4 + c] = v;
-                        }
-            m.pdc = up<real>(pdc.data(), pdc.size());
-            m.pd4 = up<real>(pd4.data(), pd4.size());
-        }
-        m.w_val = up<real>(d.w_val, S * d.kw);
-        m.j0 = up<real>(d.j0, nJ * 3);
-        m.jd = up<real>(d.jd, nJ * 3 * nd);
-        m.coefs = up<real>(d.coefs, size_t(d.n_markers) * 3);
-        m.prior_means = up<real>(d.prior_means, size_t(d.prior_k) * d.prior_d);
-        {
-            const size_t K = d.prior_k, D = d.prior_d, D4 = (D + 3) & ~size_t(3);
-            m.prior_d4 = int(D4);
-            std::vector<double> q4(K * D * D4, 0.0);
-            for (size_t k = 0; k < K; ++k)
-                for (size_t i = 0; i < D; ++i)
-                    for (size_t l = 0; l < D; ++l) q4[(k * D + i) * D4 + l] = d.prior_Q[(k * D + i) * D + l];
-            m.prior_Q4 = up<real>(q4.data(), q4.size());
-            std::vector<double> qt(K * D * D4, 0.0);
-            for (size_t k = 0; k < K; ++k)
-                for (size_t i = 0; i < D; ++i)
-                    for (size_t l = 0; l < D; ++l) qt[(k * D + l) * D4 + i] = d.prior_Q[(k * D + i) * D + l];
-            m.prior_Qt = up<real>(qt.data(), qt.size());
-        }
-        m.prior_nlw = up<real>(d.prior_neglogw, d.prior_k);
-        {
-            std::vector<int> ids(d.prior_d);
-            for (int i = 0; i < d.prior_d; ++i) ids[i] = d.prior_ids ? d.prior_ids[i] : d.prior_off + i;
-            m.prior_ids = up<int>(ids.data(), ids.size());
-        }
-        m.free1 = up<int>(d.free1, d.n_free1);
-        m.free2 = up<int>(d.free2, d.n_free2);
-        {   // image of the staged shared-memory tables, as the CUDA library builds it (mosh2.cu DevModel::build)
-            const mosh2::Dims dd = mosh2::make_dims(m);
-            mosh2::Work<real, false> w{};
-            mosh2::Arena S{mosh2::kSmemHeader}, G{0};
-            mosh2::carve<real, false>(w, dd, m, S, G);
-            std::vector<unsigned char> img(w.stage_bytes, 0);
-            const int *isrc[6] = {m.parents, m.fk_order, m.w_joint, m.free1, m.free2, m.prior_ids};
-            const real *rsrc[9] = {m.w_val, m.v0, m.coefs, m.j0, m.hands_mean, m.prior_means, m.prior_nlw, m.jd, m.hct};
-            mosh2::stage_image(w, dd, m.hct_size, m.n_hand_full, [&](uint32_t ofs, int id, size_t n) {
-                if (id < 6) std::memcpy(img.data() + ofs, isrc[id], n * sizeof(int));
-                else std::memcpy(img.data() + ofs, rsrc[id - 6], n * sizeof(real));
-            });
-            m.stage_blob = up<unsigned char>(img.data(), img.size());
+        m.tile_markers = 20;
+        m.dev_no_tc = 1;                             // the host build runs the CUDA-core formulation
+        d = mosh2::make_dims(m);
+        mosh2::Arena S{mosh2::kSmemHeader}, G{0};
+        mosh2::carve<real, false>(w, d, m, S, G);
+        smem_bytes = S.off;
+        smem_raw.resize(S.off + 128);
+
+        const size_t F = n_frames, M = desc.n_markers, nd = desc.n_dmpl;
+        fullpose.resize(F * 3 * desc.n_joints); pose.resize(F * desc.p_red); trans.resize(F * 3); dmpls.resize(F * nd + 1);
+        mk.resize(F * M * 3); errs.resize(F * mosh2::N_ERR); status.resize(F); counters.resize(F * 4);
+        job.n_frames = n_frames;
+        job.fullpose = fullpose.data(); job.pose = pose.data(); job.trans = trans.data();
+        job.dmpls = nd ? dmpls.data() : nullptr; job.markers_sim = mk.data(); job.errs = errs.data();
+        job.status = status.data(); job.counters = counters.data();
+        job.opt = mosh2_host::options(opt);
+    }
+
+    // chunks [c0, c1) one after the other, each on a zeroed shared-memory buffer
+    void run_chunks(int c0, int c1) {
+        char *smem_base = smem_raw.data() + ((32 - (reinterpret_cast<uintptr_t>(smem_raw.data()) & 31)) & 31);
+        mosh2::m2_smem_ref() = reinterpret_cast<unsigned char *>(smem_base);
+        for (int c = c0; c < c1; ++c) {
+            std::memset(smem_base, 0, smem_bytes + 64);
+            mosh2::Cta cta{0, 1};
+            mosh2::Solver<real, false> s(m, job, w, d, cta);
+            s.run_chunk(c);
         }
     }
 };
@@ -120,134 +88,54 @@ struct HostModel {
 template <class real>
 int run(const mosh2_model_desc *desc, const mosh2_options *opt, int n_frames, const double *obs, const uint8_t *vis,
         const mosh2_schedule *sched, const mosh2_result *res, int n_seq = 1, const int *seq_counts = nullptr, bool resume_all = false) {
-    const int chunk_len = sched ? sched->chunk_len : 0, warmup = sched ? sched->chunk_warmup : 0;
     if (!seq_counts) seq_counts = &n_frames;
-    HostModel<real> hm;
-    hm.build(*desc);
+    Emu<real> e(*desc, opt, n_frames);
     const size_t F = n_frames, M = desc->n_markers, PF = size_t(3) * desc->n_joints, PR = desc->p_red, nd = desc->n_dmpl;
     std::vector<real> o(F * M * 3);
     for (size_t i = 0; i < o.size(); ++i) o[i] = real(obs[i]);
-    std::vector<real> fullpose(F * PF), pose(F * PR), trans(F * 3), dmpls(F * nd + 1), mk(F * M * 3), errs(F * mosh2::N_ERR);
-    mosh2::Job<real> job{};
-    job.n_frames = n_frames;
-    const int wu = warmup > 0 ? warmup : 0;
-    const int wf = (!sched || sched->warmup_full < 0 || sched->warmup_full > wu) ? wu : sched->warmup_full;
-    const int first_extra = (sched && sched->first_extra > 0 && chunk_len > 0 && wu > 0) ? sched->first_extra : 0;
-    std::vector<int> tab = mosh2_host::chunk_table(seq_counts, n_seq, chunk_len, wu, wf, first_extra);
+    const mosh2_host::Schedule s = mosh2_host::schedule(sched);
+    std::vector<int> tab = mosh2_host::chunk_table(seq_counts, n_seq, s.chunk_len, s.warmup, s.warm_full, s.first_extra);
+    int totals[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    mosh2::Job<real> &job = e.job;
     job.n_chunks = int(tab.size() / mosh2::kChunkRec);
     job.chunk_tab = tab.data();
-    job.chunk_ids = nullptr; job.warm_x = nullptr; job.warm_f = nullptr; job.merge_tol = 0;
     job.obs = o.data(); job.vis = vis;
-    job.fullpose = fullpose.data(); job.pose = pose.data(); job.trans = trans.data();
-    job.dmpls = nd ? dmpls.data() : nullptr; job.markers_sim = mk.data(); job.errs = errs.data();
-    std::vector<int> status(F, 0), counters(F * 4, 0);
-    job.status = status.data(); job.counters = counters.data();
-    int totals[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     job.totals = totals;
-    job.prof = nullptr;
-    job.gws = nullptr; job.gws_stride = 0;
-    mosh2::Options &q = job.opt;
-    q.wt_data = opt->wt_data; q.wt_poseB = opt->wt_poseB; q.wt_poseH = opt->wt_poseH; q.wt_velo = opt->wt_velo;
-    q.wt_dmpl = opt->wt_dmpl; q.wt_annealing = opt->wt_annealing; q.wt_extrap = opt->wt_extrap_dmpl;
-    q.num_train_markers = opt->num_train_markers; q.delta_0 = opt->delta_0; q.e3_first = opt->e3_first; q.e3 = opt->e3;
-    q.maxiter = opt->maxiter; q.optimize_fingers = opt->optimize_fingers; q.optimize_dynamics = opt->optimize_dynamics;
-    q.wt_poseF = opt->wt_poseF; q.wt_expr = opt->wt_expr; q.optimize_face = opt->optimize_face;
-
-    hm.m.tile_markers = 20;
-    hm.m.dev_no_tc = 1;                          // the host build runs the CUDA-core formulation
-    const mosh2::Dims d = mosh2::make_dims(hm.m);
-    mosh2::Work<real, false> w{};
-    mosh2::Arena S0{mosh2::kSmemHeader}, G0{0};
-    mosh2::carve<real, false>(w, d, hm.m, S0, G0);
-    if (std::getenv("MOSH2_EMU_PLAN")) {        // development aid: shared-memory footprint of this model
-        for (int tile : {20, 10}) {
-            hm.m.tile_markers = tile;
-            hm.m.dev_no_tc = sizeof(real) == 4 ? 0 : 1;   // what the GPU launch would lay out
-            const mosh2::Dims dd = mosh2::make_dims(hm.m);
-            mosh2::Work<real, false> ww{};
-            mosh2::Arena Sa{mosh2::kSmemHeader}, Ga{0};
-            mosh2::carve<real, false>(ww, dd, hm.m, Sa, Ga);
-            std::fprintf(stderr, "plan: sizeof(real)=%zu tile=%d smem=%zu bytes (limit %d)\n", sizeof(real), tile, Sa.off, 227 * 1024);
-            std::fprintf(stderr, "      A=%u Lm=%u Xhi=%u Xlo=%u Jt=%u Jf=%u Loc=%u MtR=%u u=%u dtg=%u Linv=%u tc_ok=%d\n", ww.A.ofs, ww.Lm.ofs, ww.Xhi.ofs,
-                         ww.Xlo.ofs, ww.Jt.ofs, ww.Jf.ofs, ww.Loc.ofs, ww.MtR.ofs, ww.u.ofs, ww.dtg.ofs, ww.Linv.ofs, ww.tc_ok);
-        }
-        hm.m.tile_markers = 20;
-        hm.m.dev_no_tc = 1;
-    }
-    std::vector<char> smem_raw(S0.off + 128);
-    char *smem_base = smem_raw.data() + ((32 - (reinterpret_cast<uintptr_t>(smem_raw.data()) & 31)) & 31);
-    mosh2::m2_smem_ref() = reinterpret_cast<unsigned char *>(smem_base);
-    for (int c = 0; c < job.n_chunks; ++c) {
-        std::memset(smem_base, 0, S0.off + 64);
-        mosh2::Cta cta{0, 1};
-        mosh2::Solver<real, false> s(hm.m, job, w, d, cta);
-        s.run_chunk(c);
-    }
+    e.run_chunks(0, job.n_chunks);
     if (resume_all) {       // boundary repair of every chunk, in order: chunk c continues from the rows chunk c-1 emitted
         for (int c = 1; c < job.n_chunks; ++c) {
             tab[size_t(c) * mosh2::kChunkRec + 3] = -1;
-            std::memset(smem_base, 0, S0.off + 64);
-            mosh2::Cta cta{0, 1};
-            mosh2::Solver<real, false> s(hm.m, job, w, d, cta);
-            s.run_chunk(c);
+            e.run_chunks(c, c + 1);
         }
     }
     auto conv = [](double *dst, const std::vector<real> &src, size_t n) {
         if (dst) for (size_t i = 0; i < n; ++i) dst[i] = double(src[i]);
     };
-    conv(res->fullpose, fullpose, F * PF);
-    conv(res->pose, pose, F * PR);
-    conv(res->trans, trans, F * 3);
-    if (nd) conv(res->dmpls, dmpls, F * nd);
-    conv(res->markers_sim, mk, F * M * 3);
-    conv(res->errs, errs, F * mosh2::N_ERR);
-    if (res->status) std::memcpy(res->status, status.data(), F * sizeof(int));
-    if (res->counters) std::memcpy(res->counters, counters.data(), F * 4 * sizeof(int));
+    conv(res->fullpose, e.fullpose, F * PF);
+    conv(res->pose, e.pose, F * PR);
+    conv(res->trans, e.trans, F * 3);
+    if (nd) conv(res->dmpls, e.dmpls, F * nd);
+    conv(res->markers_sim, e.mk, F * M * 3);
+    conv(res->errs, e.errs, F * mosh2::N_ERR);
+    if (res->status) std::memcpy(res->status, e.status.data(), F * sizeof(int));
+    if (res->counters) std::memcpy(res->counters, e.counters.data(), F * 4 * sizeof(int));
     return 0;
 }
 
 // linearise mode (mosh2_job_linearize): every frame evaluated / linearised at the caller's state, float64
 int run_lin(const mosh2_model_desc *desc, const mosh2_options *opt, int n_frames, const double *obs, const uint8_t *vis,
             int step, int build, const double *x, const mosh2_lin_out *out) {
-    typedef double real;
-    HostModel<real> hm;
-    hm.build(*desc);
-    const size_t F = n_frames, M = desc->n_markers, PF = size_t(3) * desc->n_joints, PR = desc->p_red, nd = desc->n_dmpl;
-    const size_t NX = 3 + PR + nd, n = step == 2 ? desc->n_free2 : desc->n_free1;
-    std::vector<real> fullpose(F * PF), pose(F * PR), trans(F * 3), dmpls(F * nd + 1), mk(F * M * 3), errs(F * mosh2::N_ERR);
-    std::vector<real> A(F * n * n), g(F * n), J(F * 3 * M * n), r(F * 3 * M), vp(F * 9 * M);
-    mosh2::Job<real> job{};
-    job.n_frames = n_frames; job.n_chunks = n_frames;
+    Emu<double> e(*desc, opt, n_frames);
+    const size_t F = n_frames, M = desc->n_markers, n = step == 2 ? desc->n_free2 : desc->n_free1;
+    std::vector<double> A(F * n * n), g(F * n), J(F * 3 * M * n), r(F * 3 * M), vp(F * 9 * M);
+    mosh2::Job<double> &job = e.job;
+    job.n_chunks = n_frames;
     job.obs = obs; job.vis = vis;
-    job.fullpose = fullpose.data(); job.pose = pose.data(); job.trans = trans.data();
-    job.dmpls = nd ? dmpls.data() : nullptr; job.markers_sim = mk.data(); job.errs = errs.data();
-    std::vector<int> status(F, 0), counters(F * 4, 0);
-    job.status = status.data(); job.counters = counters.data();
     job.lin_mode = build ? 2 : 1; job.lin_step = step; job.lin_x = x;
     job.lin_A = A.data(); job.lin_g = g.data(); job.lin_J = J.data(); job.lin_r = r.data(); job.lin_vp = vp.data();
-    mosh2::Options &q = job.opt;
-    q.wt_data = opt->wt_data; q.wt_poseB = opt->wt_poseB; q.wt_poseH = opt->wt_poseH; q.wt_velo = opt->wt_velo;
-    q.wt_dmpl = opt->wt_dmpl; q.wt_annealing = opt->wt_annealing; q.wt_extrap = opt->wt_extrap_dmpl;
-    q.num_train_markers = opt->num_train_markers; q.delta_0 = opt->delta_0; q.e3_first = opt->e3_first; q.e3 = opt->e3;
-    q.maxiter = opt->maxiter; q.optimize_fingers = opt->optimize_fingers; q.optimize_dynamics = opt->optimize_dynamics;
-    q.wt_poseF = opt->wt_poseF; q.wt_expr = opt->wt_expr; q.optimize_face = opt->optimize_face;
-    hm.m.tile_markers = 20;
-    hm.m.dev_no_tc = 1;
-    const mosh2::Dims d = mosh2::make_dims(hm.m);
-    mosh2::Work<real, false> w{};
-    mosh2::Arena S0{mosh2::kSmemHeader}, G0{0};
-    mosh2::carve<real, false>(w, d, hm.m, S0, G0);
-    std::vector<char> smem_raw(S0.off + 128);
-    char *smem_base = smem_raw.data() + ((32 - (reinterpret_cast<uintptr_t>(smem_raw.data()) & 31)) & 31);
-    mosh2::m2_smem_ref() = reinterpret_cast<unsigned char *>(smem_base);
-    for (int f = 0; f < n_frames; ++f) {
-        std::memset(smem_base, 0, S0.off + 64);
-        mosh2::Cta cta{0, 1};
-        mosh2::Solver<real, false> s(hm.m, job, w, d, cta);
-        s.run_chunk(f);
-    }
-    auto back = [](double *dst, const std::vector<real> &src) { if (dst) std::memcpy(dst, src.data(), src.size() * sizeof(double)); };
-    back(out->errs, errs); back(out->markers_sim, mk); back(out->r, r); back(out->vp, vp);
+    e.run_chunks(0, n_frames);
+    auto back = [](double *dst, const std::vector<double> &src) { if (dst) std::memcpy(dst, src.data(), src.size() * sizeof(double)); };
+    back(out->errs, e.errs); back(out->markers_sim, e.mk); back(out->r, r); back(out->vp, vp);
     if (build) { back(out->A, A); back(out->g, g); back(out->J, J); }
     return 0;
 }
